@@ -7,7 +7,8 @@ i.e. 501 Dynamics.forward calls.  Arms:
                     `e2e`: the same through the public API from pinned HOST tensors (H2D + D2H inside the region).
   --impl reference  the reference algorithm's CPU implementation (oracle port; the Python reference cannot travel
                     to the GPU box) on the host cores, bounded sample per step.
-Prints ONE JSON line (rank 0).
+Prints ONE JSON line (rank 0). `--dump-outputs DIR` also writes what the last timed step returned (see dump_outputs), so
+that two builds can be compared output for output on identical seeded inputs.
 """
 import argparse
 import json
@@ -41,7 +42,28 @@ def parse_args():
                          "ranks (distributed.sample_chain_sharded: same result as on one GPU)")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu-baseline", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="native arm: after the timed steps, write rank 0's results of the last timed step as DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl != "native":
+        ap.error("--dump-outputs applies to the native arm")
+    return args
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes each tensor as out_dir/<name>.npy in float32. Every workload's results fit the limit whole, so nothing is
+    sampled: a larger total is refused rather than silently cut."""
+    import numpy as np
+    host = {name: t.detach().to(torch.float32).cpu().numpy() for name, t in arrays.items()}
+    total = sum(a.nbytes for a in host.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise SystemExit(f"--dump-outputs: {total} bytes exceed the {DUMP_LIMIT_BYTES}-byte limit")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in host.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def measured_peaks():
@@ -366,6 +388,13 @@ def main():
         d2h = ch.numel() * ch.element_size() + nm.numel() * nm.element_size()
         e2e = {"value": mols / (e2e_ms * 1e-3), "unit": "molecules/s", "h2d_bytes_per_step": h2d,
                "d2h_bytes_per_step": d2h, "ms_per_step": e2e_ms / args.steps}
+
+    if args.dump_outputs and rank == 0:
+        # chain: EDM.sample_chain of the kernel-resident arm, (1,B,N,3+F); e2e_*: DDPM.sample_chain of the end-to-end arm
+        outputs = {"chain": chain}
+        if e2e is not None:
+            outputs.update(e2e_chain=ch, e2e_node_mask=nm)
+        dump_outputs(args.dump_outputs, outputs)
 
     # ---------------- roofline of the dominant kernel (GCL edge kernel) ------------------------------------
     peaks = measured_peaks()

@@ -333,6 +333,23 @@ def golden_xyz(ns):
              text=torch.tensor(list(blob), dtype=torch.uint8), offsets=torch.tensor(offs))
 
 
+def golden_reference_edm(ns, spec, seed=3):
+    """The EDM of a freshly constructed reference DDPM (lightning.py:41-112): its state_dict keys in order, their shapes,
+    a sha256 of the values and its T. `accelerate()` replaces exactly this module, so the test rebuilds it from these
+    records; the native DDPM draws the same values for the same seed (asserted here)."""
+    from difflinker_b200.ddpm import DDPM as NativeDDPM
+    hp = synthetic.model_hparams(spec)
+    torch.manual_seed(seed)
+    ref = ns.lightning.DDPM(**hp, data_path=None, batch_size=2, lr=1e-4, torch_device='cpu', test_epochs=1,
+                            n_stability_samples=1)
+    sd = ref.edm.state_dict()
+    torch.manual_seed(seed)
+    mine = NativeDDPM(**hp).edm.state_dict()
+    assert list(mine) == list(sd) and all(torch.equal(mine[k], v) for k, v in sd.items()), "native EDM construction diverged"
+    save("ref_edm_small_fc", dict(kind="reference_edm", spec=spec.name, seed=seed, T=ref.edm.T, cls=type(ref.edm).__name__,
+                                  keys=list(sd), shapes=[list(v.shape) for v in sd.values()], sha=state_sha(sd)))
+
+
 def golden_schedules():
     ns = load_reference()
     arrs = {}
@@ -353,6 +370,7 @@ def main():
     small = synthetic.WorkloadSpec("small_fc", B=3, N=12, n_min=7, l_min=2, l_max=4, F=8, L=2, T=20, seed=11)
     golden_dynamics(ns, "dyn_small_fc", small, 3, seed=0)
     golden_dynamics(ns, "dyn_small_fc_tscalar", small, 3, seed=1, t_scalar=True)
+    golden_reference_edm(ns, small)
     golden_dynamics(ns, "dyn_cfg1", S["cfg1_plumbing"], 4, seed=0)
     geom = synthetic.WorkloadSpec("small_geom", B=5, N=23, n_min=11, l_min=1, l_max=9, F=9, L=3, T=20, seed=12,
                                   anchors_context=True)

@@ -1,5 +1,6 @@
 """Shared test plumbing: golden-vector loading, seeded model construction (weights are reproduced from the seed
 and verified by sha256 -- see oracle/make_golden.py), oracle configs."""
+import contextlib
 import hashlib
 import json
 import os
@@ -11,6 +12,21 @@ from difflinker_b200 import synthetic
 from oracle import difflinker_oracle as orc
 
 GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
+GOLDEN_THREADS = 8          # oracle/make_golden*.py generate the fixtures under torch.set_num_threads(8)
+
+
+@contextlib.contextmanager
+def golden_threads():
+    """Replays a fixture on the CPU with the torch thread count it was generated with. torch's CPU results depend in the last
+    bits on the intra-op thread count, and a chain of reverse steps amplifies those bits beyond the fixtures' tolerance (on a
+    16-core host the oracle chains end 1 ulp of coordinates near 2e4 away from the reference's; at 8 threads, bit-exact)."""
+    saved = torch.get_num_threads()
+    torch.set_num_threads(GOLDEN_THREADS)
+    try:
+        yield
+    finally:
+        torch.set_num_threads(saved)
+
 
 EXTRA_SPECS = {
     "small_fc": synthetic.WorkloadSpec("small_fc", B=3, N=12, n_min=7, l_min=2, l_max=4, F=8, L=2, T=20, seed=11),

@@ -740,3 +740,28 @@ def test_batch_slices_reproduce_the_single_gpu_chain(world):
         parts.append(ddpm.edm.sample_chain(**slice_sampler_inputs(kw, lo, hi), keep_frames=2, batch_slice=(lo, 7)))
     assert torch.equal(torch.cat(parts, dim=1), full)
 
+
+
+def test_bench_dumps_the_last_timed_step_reproducibly(tmp_path):
+    """`bench.py --dump-outputs DIR` writes the results of its last timed step; with the same arguments the inputs are the same
+    seeded ones, so two runs write identical arrays. `--steps` sets the number of timed sampler calls."""
+    import json, os, subprocess, sys
+    import numpy as np
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    spec = synthetic.SPECS["cfg1_plumbing"]
+    runs = []
+    for r in range(2):
+        out = tmp_path / f"run{r}"
+        res = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--workload", spec.name, "--T", "10", "--steps", "2",
+                              "--warmup", "1", "--no-cpu-baseline", "--dump-outputs", str(out)], capture_output=True, text=True,
+                             timeout=600)
+        assert res.returncode == 0, res.stderr[-3000:]
+        line = json.loads([l for l in res.stdout.splitlines() if l.startswith("{")][-1])
+        assert line["steps"] == 2 and len(line["loop_ms_device"]) == 2
+        runs.append({n: np.load(out / f"{n}.npy") for n in ("chain", "e2e_chain", "e2e_node_mask")})
+    a, b = runs
+    assert a["chain"].shape == (1, spec.B, spec.N, 3 + spec.F) and a["chain"].dtype == np.float32
+    assert a["e2e_chain"].shape == a["chain"].shape and a["e2e_node_mask"].shape == (spec.B, spec.N, 1)
+    assert np.isfinite(a["chain"]).all()
+    for n in a:
+        assert np.array_equal(a[n], b[n]), n

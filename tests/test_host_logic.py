@@ -204,18 +204,20 @@ print("ok")
 
 
 def test_accelerate_swaps_reference_edm():
-    """Whole-loop drop-in: a *reference* DDPM (live reference, build container only) gets the native EDM with
-    the same weights; strict state_dict load proves the key layout."""
-    from oracle.ref_loader import load_reference, reference_available
-    if not reference_available():
-        pytest.skip("reference checkout not present on this machine")
-    ns = load_reference()
-    spec = helpers.EXTRA_SPECS["small_fc"]
-    hp = synthetic.model_hparams(spec)
-    torch.manual_seed(3)
-    ref = ns.lightning.DDPM(**hp, data_path=None, batch_size=2, lr=1e-4, torch_device='cpu', test_epochs=1,
-                            n_stability_samples=1)
-    ref.hparams = hp                                         # the Lightning stub has no save_hyperparameters
+    """Whole-loop drop-in: a *reference* DDPM gets the native EDM with the same weights; strict state_dict load proves the
+    key layout. accelerate() reads `hparams`, `edm.state_dict()` and `edm.T` of the reference DDPM; the stand-in carries
+    the reference EDM's state_dict as recorded by oracle/make_golden.py (keys in its order, shapes, sha256 of the values
+    its constructor draws for the seed), and the seeded native DDPM reproduces those values."""
+    import types
+    meta, _ = helpers.load_golden("ref_edm_small_fc")
+    assert meta["cls"] == "EDM"
+    hp = synthetic.model_hparams(helpers.spec_by_name(meta["spec"]))
+    torch.manual_seed(meta["seed"])
+    sd = difflinker_b200.DDPM(**hp).edm.state_dict()
+    assert list(sd) == meta["keys"] and [list(v.shape) for v in sd.values()] == meta["shapes"]
+    assert helpers.state_sha(sd) == meta["sha"]
+    ref_edm = types.SimpleNamespace(state_dict=lambda: sd, T=meta["T"])
+    ref = types.SimpleNamespace(hparams=hp, edm=ref_edm)
     before = {k: v.clone() for k, v in ref.edm.state_dict().items()}
     ref.edm.T = 7
     out = difflinker_b200.accelerate(ref)

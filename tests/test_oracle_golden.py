@@ -41,7 +41,7 @@ def test_oracle_chain_matches_reference_golden(name):
     com = tpl['fragment_only_mask'] if spec.pocket else tpl['fragment_mask']   # lightning.py:441-444 (MOAD val_dataset)
     x = orc.remove_partial_mean(tpl['positions'], tpl['atom_mask'], com)
     gam = orc.gamma_table(hp['diffusion_noise_schedule'], hp['diffusion_steps'], hp['diffusion_noise_precision'])
-    with torch.no_grad():
+    with torch.no_grad(), helpers.golden_threads():
         chain = orc.edm_sample_chain(ddpm.edm.dynamics.state_dict(), helpers.oracle_cfg(hp), gam, meta["T"], x,
                                      tpl['one_hot'], tpl['atom_mask'], tpl['fragment_mask'], tpl['linker_mask'],
                                      tpl['edge_mask'], helpers.context_of(tpl, spec), keep_frames=meta["keep_frames"],
@@ -62,7 +62,7 @@ def test_oracle_inpainting_chain_matches_reference_golden():
     gam = orc.gamma_table(hp['diffusion_noise_schedule'], hp['diffusion_steps'], hp['diffusion_noise_precision'])
     ocfg = helpers.oracle_cfg(hp)
     ocfg.centering = True                                                                   # lightning.py:99
-    with torch.no_grad():
+    with torch.no_grad(), helpers.golden_threads():
         chain = orc.inpainting_sample_chain(ddpm.edm.dynamics.state_dict(), ocfg, gam, meta["T"], x, data['one_hot'],
                                             data['atom_mask'], data['fragment_mask'], data['linker_mask'],
                                             data['edge_mask'], data['fragment_mask'], keep_frames=meta["keep_frames"],
