@@ -9,6 +9,9 @@ DL_OK, DL_NAN_DETECTED = 0, 1
 GRAPH_TYPES = {"FC": 0, "4A": 1, "FC-4A": 2, "FC-10A-4A": 3}
 EDGE_IMPLS = {"auto": 0, "simt": 1, "tcgen05": 2}
 SAMPLER_LINKER, SAMPLER_INPAINT = 0, 1
+# dl_diffusion_loss: rows of the per-molecule coefficient table and columns of the per-molecule terms
+LOSS_COEFS = ("t", "alpha_t", "sigma_t", "alpha_1", "sigma2_1", "log_inv_sigma_1")
+LOSS_TERMS = ("error_t", "noise", "log_p_x", "log_p_h", "kl_prior", "n_linker")
 
 
 class DLConfig(C.Structure):
@@ -44,6 +47,7 @@ SYMBOLS = {
     "dl_sample_chain": (_I32, [_P, _I32, _I32, _I32, _I32, _I32, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P]),
     "dl_sample_chain_rng": (_I32, [_P, _I32, _I32, _I32, _I32, _I32, _P, _P, _P, _P, _P, _P, C.c_uint64, C.c_uint64, _P, _P, _P, _P,
                                    _P, _P]),
+    "dl_diffusion_loss": (_I32, [_P, _I32, _I32, _P, _P, _P, _P, _P, _P, _P, _P, C.c_uint64, C.c_uint64, _P, _P, _P, _P, _P]),
     "dl_set_noise_slice": (_I32, [_P, _I32, _I32]),
     "dl_noise_fill": (_I32, [_P, _I32, _I32, _I32, C.c_uint64, C.c_uint64, _P, _P, _P]),
     "dl_sample_chain_host": (_I32, [_P, _I32, _I32, _I32, _I32, _I32, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P]),

@@ -8,7 +8,7 @@ PKG_DIR = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(PKG_DIR, "csrc")
 LIB_PATH = os.path.join(PKG_DIR, "libdifflinker_b200.so")
 SOURCES = ["dl_engine.cu", "output_stage.cu"]
-HEADERS = ["common.cuh", "size_gnn.cuh", "kernels_simt.cuh", "kernels_tc.cuh", "kernels_node_tc.cuh", "kernels_edge_v3.cuh", os.path.join("..", "..", "include", "difflinker_b200.h")]
+HEADERS = ["common.cuh", "size_gnn.cuh", "kernels_simt.cuh", "kernels_tc.cuh", "kernels_node_tc.cuh", "kernels_edge_v3.cuh", "diffusion_loss.cuh", os.path.join("..", "..", "include", "difflinker_b200.h")]
 
 
 def nvcc_path():

@@ -19,6 +19,7 @@
 #include "kernels_tc.cuh"
 #include "kernels_node_tc.cuh"
 #include "kernels_edge_v3.cuh"
+#include "diffusion_loss.cuh"
 
 using namespace dl;
 
@@ -45,6 +46,7 @@ struct Workspace {
   int B = 0, N = 0;
   float *nm = nullptr, *x0 = nullptr, *xa = nullptr, *xb = nullptr, *h = nullptr, *ABg = nullptr, *ABc = nullptr,
         *agg = nullptr, *z = nullptr, *ABgmax = nullptr, *ABcmax = nullptr, *eps = nullptr;
+  float* eps_hat = nullptr;   // dl_diffusion_loss: the Dynamics.forward output on z_t (z holds z_t, eps holds eps_t)
   int* cls = nullptr;
   // cut-off graphs on the tcgen05 path: per-row neighbour lists and packed tile records of the current call (k_nbr)
   int *nbr = nullptr, *recs = nullptr, *xrecs = nullptr, *n_recs = nullptr;
@@ -239,7 +241,7 @@ dl_status ensure_workspace(dl_engine* e, int B, int N) {
   dl_status s;
 #define WSA(field, cnt) if ((s = dev_alloc(ws, &ws.field, (cnt))) != DL_OK) return s
   WSA(nm, n); WSA(x0, n * 3); WSA(xa, n * 3); WSA(xb, n * 3); WSA(h, n * H); WSA(ABg, n * 2 * H); WSA(ABc, n * 2 * H);
-  WSA(agg, n * H); WSA(z, n * xd); WSA(eps, n * xd); WSA(cls, n); WSA(x04, n); WSA(xa4, n); WSA(xb4, n); WSA(ABgmax, n * 2); WSA(ABcmax, n * 2);
+  WSA(agg, n * H); WSA(z, n * xd); WSA(eps, n * xd); WSA(eps_hat, n * xd); WSA(cls, n); WSA(x04, n); WSA(xa4, n); WSA(xb4, n); WSA(ABgmax, n * 2); WSA(ABcmax, n * 2);
   WSA(rowidx, n); WSA(colidx, n); WSA(xrowidx, n); WSA(nr, B); WSA(nc, B); WSA(nxr, B); WSA(n_items, 1);
   WSA(xmols, B); WSA(n_xmols, 1); WSA(items, n); WSA(xitems, n); WSA(n_xitems, 1); WSA(tile_ctr, 64);
   if (e->use_tc && e->cfg.graph_type != 0) { WSA(nbr, n * N); WSA(recs, n * CUT_REC); WSA(xrecs, n * CUT_REC); WSA(n_recs, 2); }
@@ -860,6 +862,48 @@ dl_status dl_sample_chain_rng(dl_engine* e, int32_t sampler, int32_t B, int32_t 
   if (offset_consumed) *offset_consumed = (uint64_t)(T + 2) * q.per_draw;
   return sample_chain_impl(e, sampler, B, N, T, keep_frames, xh, node_mask, fragment_mask, linker_mask, edge_mask, context, nullptr,
                            &q, coef, norm, chain, nan_flags, stream);
+}
+
+dl_status dl_diffusion_loss(dl_engine* e, int32_t B, int32_t N, const float* xh, const int8_t* node_mask,
+                            const float* fragment_mask, const float* linker_mask, const int8_t* edge_mask,
+                            const float* context, const float* coef, const float* eps, uint64_t seed, uint64_t offset,
+                            uint64_t* offset_consumed, const float* norm, float* terms, int32_t* nan_flags, void* stream) {
+  dl_status s = check_shapes(e, B, N);
+  if (s != DL_OK) return s;
+  if (e->cfg.centering) { set_err("dl_diffusion_loss: inpainting models (centering = 1) are not supported"); return DL_ERR_UNSUPPORTED; }
+  if (!xh || !node_mask || !fragment_mask || !linker_mask || !coef || !norm || !terms) { set_err("null argument"); return DL_ERR_INVALID; }
+  if (!e->cfg.condition_time) { set_err("dl_diffusion_loss needs a time-conditioned model (condition_time = 1)"); return DL_ERR_UNSUPPORTED; }
+  if (e->cfg.context_node_nf > 0 && !context) { set_err("context required (context_node_nf=%d)", e->cfg.context_node_nf); return DL_ERR_INVALID; }
+  if (!eps && offset % 4 != 0) { set_err("philox offset must be a multiple of 4 (torch.Generator.get_offset())"); return DL_ERR_INVALID; }
+  if (!eps && e->slice_B_full > 0) { set_err("dl_diffusion_loss draws the whole batch: switch the noise slice off first"); return DL_ERR_INVALID; }
+  CK(cudaSetDevice(e->cfg.device));
+  cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+  if ((s = ensure_workspace(e, B, N)) != DL_OK) return s;
+  Workspace& ws = e->ws;
+  const int n = B * N, xd = 3 + e->cfg.in_node_nf;
+  NoiseRng q{};
+  if (!eps) q = make_rng(e, B, N, seed, offset);
+  if (offset_consumed) *offset_consumed = eps ? 0 : (uint64_t)q.per_draw;
+  CK(cudaEventRecord(e->ev_t0, st));
+  if (nan_flags) CK(cudaMemsetAsync(nan_flags, 0, B * sizeof(int32_t), st));
+  TIMED("k_qsample", st, (k_qsample<<<(n * xd + 255) / 256, 256, 0, st>>>(n, N, xd, xh, fragment_mask, linker_mask, eps, q, coef,
+                                                                          ws.z, ws.eps)));
+  LAUNCH_CHECK();
+  e->launches += 1;
+  if ((s = build_plan(e, B, N, node_mask, linker_mask, edge_mask, st)) != DL_OK) return s;
+  FwdIO io;
+  io.xh = ws.z; io.t = coef + DL_LOSS_T * B; io.t_numel = B; io.out = ws.eps_hat; io.node_mask = node_mask;
+  io.linker_mask = linker_mask; io.edge_mask = edge_mask; io.context = context; io.nan_flags = nan_flags;
+  if ((s = enqueue_forward(e, B, N, io, st)) != DL_OK) return s;
+  LossArgs la{};
+  la.N = N; la.F = e->cfg.in_node_nf; la.xh = xh; la.z = ws.z; la.eps = ws.eps; la.out = ws.eps_hat; la.lm = linker_mask;
+  la.coef = coef; la.norm1 = norm[1]; la.bias1 = norm[2]; la.terms = terms;
+  TIMED("k_diffusion_loss", st, (k_diffusion_loss<<<B, LOSS_THREADS, 0, st>>>(la)));
+  LAUNCH_CHECK();
+  e->launches += 1;
+  CK(cudaEventRecord(e->ev_t1, st));
+  g_times.collect(st);
+  return DL_OK;
 }
 
 dl_status dl_set_noise_slice(dl_engine* e, int32_t B_full, int32_t b0) {

@@ -6,7 +6,8 @@ Two ways in:
     (`edm.gamma.gamma`, `edm.dynamics.dynamics....`), for environments without pytorch_lightning;
   * `accelerate(ddpm)` -- swaps the `.edm` of an existing *reference* DDPM (e.g. one returned by
     `DDPM.load_from_checkpoint`) for the native one in place, so generate.py / sample.py run unchanged.
-Training, datasets, metrics and visualisation are out of scope (SURVEY.md section 2).
+`DDPM.forward(data, training=False)`, `validation_step` and `test_step` (lightning.py:148-268) evaluate the diffusion
+loss; training (backward, optimiser), datasets, metrics and visualisation are out of scope (SURVEY.md section 2).
 """
 import torch
 import torch.nn as nn
@@ -86,8 +87,71 @@ def sample_chain(model, data, sample_fn=None, keep_frames=None):
     return chain, kw['node_mask']
 
 
+def loss_forward(model, data):
+    """Body of DDPM.forward(data, training=False) (lightning.py:148-199). `model` needs .anchors_context, .train_dataset,
+    .inpainting, .center_of_mass and .edm. NB the pocket switch tests train_dataset here, where the sampler tests
+    val_dataset (lightning.py:441)."""
+    x = data['positions']
+    h = data['one_hot']
+    node_mask = data['atom_mask']
+    edge_mask = data['edge_mask']
+    anchors = data['anchors']
+    fragment_mask = data['fragment_mask']
+    linker_mask = data['linker_mask']
+    if model.anchors_context:
+        context = torch.cat([anchors, fragment_mask], dim=-1)
+    else:
+        context = fragment_mask
+    moad = type(getattr(model, 'train_dataset', None)).__name__ == 'MOADDataset'
+    if moad:
+        fragment_only_mask = data['fragment_only_mask']
+        pocket_only_mask = fragment_mask - fragment_only_mask
+        if model.anchors_context:
+            context = torch.cat([anchors, fragment_only_mask, pocket_only_mask], dim=-1)
+        else:
+            context = torch.cat([fragment_only_mask, pocket_only_mask], dim=-1)
+    if model.inpainting:
+        center_of_mass_mask = node_mask
+    elif moad and model.center_of_mass == 'fragments':
+        center_of_mass_mask = data['fragment_only_mask']
+    elif model.center_of_mass == 'fragments':
+        center_of_mass_mask = fragment_mask
+    elif model.center_of_mass == 'anchors':
+        center_of_mass_mask = anchors
+    else:
+        raise NotImplementedError(model.center_of_mass)
+    x = utils.remove_partial_mean_with_mask(x, node_mask, center_of_mass_mask)
+    # (the reference's assert_partial_mean_zero_with_mask is a host-synchronising check of the line above; not repeated)
+    return model.edm.forward(x=x, h=h, node_mask=node_mask, fragment_mask=fragment_mask, linker_mask=linker_mask,
+                             edge_mask=edge_mask, context=context)
+
+
+def step_metrics(model, data):
+    """The dict validation_step / test_step return (lightning.py:228-268)."""
+    delta_log_px, kl_prior, loss_term_t, loss_term_0, l2_loss, noise_t, noise_0 = model.forward(data, training=False)
+    vlb_loss = kl_prior + loss_term_t + loss_term_0 - delta_log_px
+    if model.loss_type == 'l2':
+        loss = l2_loss
+    elif model.loss_type == 'vlb':
+        loss = vlb_loss
+    else:
+        raise NotImplementedError(model.loss_type)
+    return {
+        'loss': loss,
+        'delta_log_px': delta_log_px,
+        'kl_prior': kl_prior,
+        'loss_term_t': loss_term_t,
+        'loss_term_0': loss_term_0,
+        'l2_loss': l2_loss,
+        'vlb_loss': vlb_loss,
+        'noise_t': noise_t,
+        'noise_0': noise_0
+    }
+
+
 class DDPM(nn.Module):
-    """Hyper-parameter-compatible stand-in for the Lightning module (sampling API only)."""
+    """Hyper-parameter-compatible stand-in for the Lightning module: sampling, and the evaluation steps
+    (validation_step / test_step)."""
     train_dataset = None
     val_dataset = None
     test_dataset = None
@@ -122,8 +186,20 @@ class DDPM(nn.Module):
     def sample_chain(self, data, sample_fn=None, keep_frames=None):
         return sample_chain(self, data, sample_fn=sample_fn, keep_frames=keep_frames)
 
-    def forward(self, *a, **k):
-        raise NotImplementedError("training is outside the difflinker_b200 hot path")
+    def forward(self, data, training):
+        """DDPM.forward (lightning.py:148-199): the diffusion objective of a collated batch through EDM.forward.
+        Evaluation only (training=False, as validation_step / test_step call it)."""
+        if training:
+            raise NotImplementedError("DDPM.forward(training=True): no backward pass on the native path")
+        return loss_forward(self, data)
+
+    def validation_step(self, data, *args):
+        """lightning.py:228-247 (without Lightning's logging)."""
+        return step_metrics(self, data)
+
+    def test_step(self, data, *args):
+        """lightning.py:249-268."""
+        return step_metrics(self, data)
 
     @classmethod
     def load_from_checkpoint(cls, checkpoint_path, map_location=None, strict=True, **overrides):

@@ -8,6 +8,7 @@ torch seed produces the same noise stream as the reference would on that device.
 """
 import ctypes as C
 
+import numpy as np
 import torch
 import torch.nn.functional as F
 
@@ -49,8 +50,112 @@ class EDM(torch.nn.Module):
         self.noise_mode = 'reference_stream'
         self.last_loop_ms = None               # device time of the last reverse loop (CUDA events)
 
-    def forward(self, *args, **kwargs):
-        raise NotImplementedError("training (src/edm.py:41-124) is outside the difflinker_b200 hot path")
+    def forward(self, x, h, node_mask, fragment_mask, linker_mask, edge_mask, context=None):
+        """The diffusion objective of a batch (edm.py:41-124), evaluation only: one q(z_t|x,h) draw per molecule, one
+        Dynamics.forward and the loss terms, on the device. Returns the reference's tuple (delta_log_px, kl_prior,
+        loss_term_t, loss_term_0, l2_loss, noise_t, noise_0); loss_term_0 and noise_0 are the float 0. when no molecule
+        drew t = 0, and the t > 0 means are NaN when every molecule did, as in the reference. No gradients."""
+        lt = self.loss_terms(x, h, node_mask, fragment_mask, linker_mask, edge_mask, context)
+        delta_log_px = lt['delta_log_px'].mean()                                      # edm.py:46
+        l2_loss = lt['l2'].mean()                                                     # edm.py:92-93
+        kl_prior = lt['kl_prior'].mean()                                              # edm.py:96
+        t_is_zero = (lt['t_int'] == 0).squeeze().float()                              # edm.py:54-55
+        t_is_not_zero = 1 - t_is_zero
+        loss_term_t = (lt['loss_term_t'] * t_is_not_zero).sum() / t_is_not_zero.sum()  # edm.py:100-101
+        noise_t = (lt['noise'] * t_is_not_zero).sum() / t_is_not_zero.sum()           # edm.py:104-105
+        if t_is_zero.sum() > 0:                                                       # edm.py:107-120
+            loss_term_0 = (lt['loss_term_0'] * t_is_zero).sum() / t_is_zero.sum()
+            noise_0 = (lt['noise'] * t_is_zero).sum() / t_is_zero.sum()
+        else:
+            loss_term_0 = 0.
+            noise_0 = 0.
+        return delta_log_px, kl_prior, loss_term_t, loss_term_0, l2_loss, noise_t, noise_0
+
+    def draw_timesteps(self, n_samples, device):
+        """edm.py:49: the reference's own randint call on the batch's device, so the generator advances as it would."""
+        return torch.randint(0, self.T + 1, size=(n_samples, 1), device=device).float()
+
+    def loss_coefficients(self, t_int):
+        """Per-molecule scalars of EDM.forward for the timesteps `t_int` (B,1): a dict of (B,1) fp32 CPU tensors evaluated
+        with the reference's ops and shapes (edm.py:49-62, 98, 244-254, 272-280), so they round as the reference's do --
+        SNR(gamma_s - gamma_t) - 1 cancels badly near t = 0. For t_int = 0, s indexes the table at -1, which wraps to its
+        last entry as in the reference; that term is masked out later."""
+        gamma = self._cpu_schedule()
+        t_int = t_int.detach().to(device='cpu', dtype=torch.float32).reshape(-1, 1)
+        n = t_int.shape[0]
+        t = t_int / self.T
+        s = (t_int - 1) / self.T
+        gamma_t, gamma_s = gamma(t), gamma(s)
+        gamma_1 = gamma(torch.ones((n, 1)))
+        sigma_1 = self.sigma(gamma_1)
+        return dict(t=t, alpha_t=self.alpha(gamma_t), sigma_t=self.sigma(gamma_t), alpha_1=self.alpha(gamma_1),
+                    sigma2_1=sigma_1 ** 2, log_inv_sigma_1=torch.log(torch.ones_like(sigma_1) / sigma_1),
+                    snr_weight=self.SNR(gamma_s - gamma_t) - 1, log_sigma_x=0.5 * gamma(torch.zeros((n, 1))))
+
+    @torch.no_grad()
+    def loss_terms(self, x, h, node_mask, fragment_mask, linker_mask, edge_mask, context=None, eps=None):
+        """Per-molecule terms of EDM.forward as (B,) tensors on x's device: t_int, error_t, l2, loss_term_t, loss_term_0,
+        kl_prior, noise, delta_log_px (before the batch reductions of edm.py:92-120; e.g. to rank molecules by their
+        loss). `eps` optionally injects the (B,N,3+F) unmasked draws."""
+        lib = _native.load_library()
+        n_samples, n_nodes = x.size(0), x.size(1)
+        dev = x.device
+        work = dev if dev.type == 'cuda' else torch.device('cuda', self.dynamics._device_index(x))
+        d = self.n_dims + self.in_node_nf
+        xn, hn = self.normalize(x, h)
+        xh = torch.cat([xn, hn], dim=2).to(device=work, dtype=torch.float32).contiguous()
+        t_int = self.draw_timesteps(n_samples, dev)                                  # edm.py:49, before the noise draw
+        on_device = (eps is None and dev.type == 'cuda' and self.noise_mode == 'reference_stream'
+                     and 'draw_noise' not in self.__dict__)
+        if not on_device:
+            if eps is None:
+                eps = self.draw_noise(1, n_samples, n_nodes, dev)[0]
+            eps = eps.to(device=work, dtype=torch.float32).contiguous()
+            assert eps.shape == (n_samples, n_nodes, d), eps.shape
+        c = self.loss_coefficients(t_int.cpu())
+        coef = torch.cat([c[k].reshape(1, -1) for k in _native.LOSS_COEFS]).to(work).contiguous()
+        eng = self.dynamics.engine(work.index)
+        self.dynamics._check_graph_type()
+        prep = lambda v, dt: None if v is None else v.detach().to(device=work, dtype=dt).contiguous()
+        nm = prep(node_mask.reshape(n_samples, n_nodes), torch.int8)
+        fm = prep(fragment_mask.reshape(n_samples, n_nodes), torch.float32)
+        lm = prep(linker_mask.reshape(n_samples, n_nodes), torch.float32)
+        em = None
+        if self.dynamics.graph_type == 'FC' and edge_mask is not None:
+            em = prep(edge_mask.reshape(-1), torch.int8)
+            assert em.numel() == n_samples * n_nodes * n_nodes
+        ctx = None if context is None else prep(
+            context.reshape(n_samples, n_nodes, self.dynamics.context_node_nf), torch.float32)   # wrong width -> raises
+        norm = (C.c_float * 3)(float(self.norm_values[0]), float(self.norm_values[1]), float(self.norm_biases[1]))
+        terms = torch.empty((n_samples, len(_native.LOSS_TERMS)), device=work, dtype=torch.float32)
+        flags = torch.zeros(n_samples, dtype=torch.int32, device=work)
+        ptr = lambda v: None if v is None else v.data_ptr()
+        with torch.cuda.device(work):
+            stream = torch.cuda.current_stream(work).cuda_stream
+            seed = offset = 0
+            if on_device:
+                gen = torch.cuda.default_generators[work.index]
+                seed, offset = gen.initial_seed() & 0xFFFFFFFFFFFFFFFF, gen.get_offset()
+            used = C.c_uint64(0)
+            st = lib.dl_diffusion_loss(eng, n_samples, n_nodes, ptr(xh), ptr(nm), ptr(fm), ptr(lm), ptr(em), ptr(ctx),
+                                       ptr(coef), ptr(eps), seed, offset, C.byref(used), norm, ptr(terms), ptr(flags), stream)
+            _native.check(st, "dl_diffusion_loss")
+            if on_device:
+                gen.set_offset(offset + used.value)     # as if randn(B,N,3) and randn(B,N,F) had run (edm.py:67)
+            if bool(flags.any().item()):             # the reference raises inside Dynamics.forward (egnn.py:441)
+                raise nan_exception_class()(flags=flags.cpu().tolist())
+        col = {k: terms[:, i] for i, k in enumerate(_native.LOSS_TERMS)}
+        on = lambda v: v.reshape(-1).to(work)
+        dof = col['n_linker'] * self.n_dims                                           # dimensionality, edm.py:402-403
+        error_t = col['error_t']
+        l2 = error_t / ((self.n_dims + self.in_node_nf) * col['n_linker'])             # edm.py:91-92
+        loss_term_t = self.T * 0.5 * on(c['snr_weight']) * error_t                    # edm.py:98-99
+        neg_log_constants = -(dof * (-on(c['log_sigma_x']) - 0.5 * np.log(2 * np.pi)))  # edm.py:272-280, 110
+        loss_term_0 = -(col['log_p_x'] + col['log_p_h']) + neg_log_constants          # edm.py:114-115, 316
+        out = dict(t_int=t_int.reshape(-1), error_t=error_t, l2=l2, loss_term_t=loss_term_t, loss_term_0=loss_term_0,
+                   kl_prior=col['kl_prior'], noise=col['noise'],
+                   delta_log_px=-dof * np.log(self.norm_values[0]))                    # edm.py:398-399
+        return {k: v.to(dev) for k, v in out.items()}
 
     # ---- scalar helpers, same names/semantics as the reference -------------------------------------------------
     def sigma(self, gamma, target_tensor=None):
@@ -75,6 +180,14 @@ class EDM(torch.nn.Module):
     def unnormalize(self, x, h):
         return x * self.norm_values[0], h * self.norm_values[1] + self.norm_biases[1]
 
+    def _cpu_schedule(self):
+        """The noise schedule with its gamma table on the host, for the scalar tables below."""
+        gamma = PredefinedNoiseSchedule.__new__(PredefinedNoiseSchedule)
+        torch.nn.Module.__init__(gamma)
+        gamma.timesteps = self.gamma.timesteps
+        gamma.gamma = torch.nn.Parameter(self.gamma.gamma.detach().cpu(), requires_grad=False)
+        return gamma
+
     def step_coefficients(self, keep_frames, n_samples=1):
         """(T+1) rows of dl_step_coef: row r is reverse step s = T-1-r (edm.py:146-163, 178-208); row T is the
         final p(x,h|z_0) step (edm.py:210-235).  Evaluated on (n_samples,1) fp32 CPU tensors exactly as the
@@ -84,10 +197,7 @@ class EDM(torch.nn.Module):
         key = (T, keep_frames, n_samples, self.gamma.gamma._version, self.gamma.gamma.data_ptr())
         if getattr(self, '_coef_cache', None) is not None and self._coef_cache[0] == key:
             return self._coef_cache[1]
-        gamma = PredefinedNoiseSchedule.__new__(PredefinedNoiseSchedule)
-        torch.nn.Module.__init__(gamma)
-        gamma.timesteps = self.gamma.timesteps
-        gamma.gamma = torch.nn.Parameter(self.gamma.gamma.detach().cpu(), requires_grad=False)
+        gamma = self._cpu_schedule()
         rows = (_native.DLStepCoef * (T + 1))()
         for r in range(T):
             s = T - 1 - r
@@ -212,6 +322,13 @@ class InpaintingEDM(EDM):
     fragments with q(z_s | z_t, x), and the centre of mass is projected out every step.
     NB the reference's positional order differs from EDM.sample_chain (edge_mask comes third): call by keyword."""
 
+    def forward(self, *args, **kwargs):
+        # no published config trains with inpainting; the objective of edm.py:466-547 is not ported
+        raise NotImplementedError("InpaintingEDM.forward (src/edm.py:466-547) is not implemented on the native path")
+
+    def loss_terms(self, *args, **kwargs):
+        raise NotImplementedError("InpaintingEDM.forward (src/edm.py:466-547) is not implemented on the native path")
+
     @staticmethod
     def _com_free(x, mask):
         """utils.sample_center_gravity_zero_gaussian_with_mask (utils.py:158-168) applied to a raw draw."""
@@ -235,10 +352,7 @@ class InpaintingEDM(EDM):
         if getattr(self, '_qcoef_key', None) == self._coef_cache[0]:
             return rows
         T = self.T
-        gamma = PredefinedNoiseSchedule.__new__(PredefinedNoiseSchedule)
-        torch.nn.Module.__init__(gamma)
-        gamma.timesteps = self.gamma.timesteps
-        gamma.gamma = torch.nn.Parameter(self.gamma.gamma.detach().cpu(), requires_grad=False)
+        gamma = self._cpu_schedule()
         for r in range(T):
             s = T - 1 - r
             s_arr = torch.full((n_samples, 1), fill_value=s)

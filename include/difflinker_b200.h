@@ -16,6 +16,7 @@
  *     sample_p_zs_given_zt_only_linker  edm.py:178-208
  *     sample_p_xh_given_z0_only_linker  edm.py:210-235
  *   InpaintingEDM.sample_chain   src/edm.py:549-612      dl_sample_chain with DL_SAMPLER_INPAINT
+ *   EDM.forward (evaluation)     src/edm.py:41-124       dl_diffusion_loss
  *   SizeClassifier.forward       src/linker_size_lightning.py:83-110  dl_sizegnn_create/.../dl_sizegnn_forward
  *   build_xae_molecule           src/molecule_builder.py:44-102       dl_bond_orders
  *   frame restore + .xyz text    generate.py:163-171, src/visualizer.py:14-31   dl_restore_frame, dl_format_xyz
@@ -173,6 +174,40 @@ dl_status dl_set_noise_slice(dl_engine* e, int32_t B_full, int32_t b0);
 /* The (n_draws,B,N,3+F) tensor the device-side stream of dl_sample_chain_rng stands for (tests, debugging). DEVICE out. */
 dl_status dl_noise_fill(dl_engine* e, int32_t n_draws, int32_t B, int32_t N, uint64_t seed, uint64_t offset, float* out,
                         uint64_t* offset_consumed, void* stream);
+
+/*
+ * The diffusion objective of EDM.forward (edm.py:41-124) for a batch, evaluation only (no backward): what
+ * DDPM.validation_step / test_step (lightning.py:228-268) compute through DDPM.forward(data, training=False).
+ *   1. q(z_t | x, h) on the linker atoms (edm.py:64-75): z_t = xh*fragment_mask + (alpha_t*xh + sigma_t*eps_t)*linker_mask,
+ *      eps_t = [randn(B,N,3), randn(B,N,F)] * linker_mask;
+ *   2. one Dynamics.forward(z_t, t) with the per-molecule t (edm.py:78-85), FC or cut-off graph;
+ *   3. per molecule, with eps_hat = out * linker_mask, the sums the loss is made of (edm.py:88-124, 244-318, 405-463).
+ *   xh          (B,N,3+F) normalised input (x/norm0, (h-bias)/norm1), DEVICE
+ *   fragment_mask, linker_mask (B,N) fp32; node_mask (B,N) int8; edge_mask, context as for dl_dynamics_forward. DEVICE
+ *   coef        (DL_LOSS_COEFS, B) fp32 DEVICE, row k = coefficient k of every molecule (DL_LOSS_T ...): t = t_int/T, alpha_t,
+ *               sigma_t of gamma(t), and alpha, sigma^2 and log(1/sigma) of gamma(1) for kl_prior -- computed by the caller
+ *               with the reference's formulas (edm.py:49-62, 251-254), so they round as the reference's do
+ *   eps         (B,N,3+F) UNMASKED standard normal draws, DEVICE, or NULL: then they are drawn on the device from (seed, offset)
+ *               in the reference's order, randn(B,N,3) then randn(B,N,F), as dl_sample_chain_rng draws one noise sample;
+ *               offset_consumed (HOST out, may be NULL) is what those two calls consume
+ *   norm        {norm_values[0], norm_values[1], norm_biases[1]} HOST
+ *   terms       (B, DL_LOSS_TERMS) fp32 DEVICE out, per molecule: DL_LOSS_ERROR_T = sum (eps_t - eps_hat)^2;
+ *               DL_LOSS_NOISE = ||eps_hat||; DL_LOSS_LOG_P_X / DL_LOSS_LOG_P_H = the x and h parts of log p(x,h|z_0)
+ *               without constants, evaluated at gamma_t (edm.py:272-318); DL_LOSS_KL_PRIOR = KL(q(z_1|x,h) || N(0,1))
+ *               (edm.py:244-270; its h part sums every row, padding included, as the reference does);
+ *               DL_LOSS_N_LINKER = number of linker atoms
+ *   nan_flags   (B) int32 DEVICE out, as for dl_dynamics_forward
+ * Sums are reduced in a fixed order: equal inputs give equal terms. Not for inpainting engines (centering = 1):
+ * DL_ERR_UNSUPPORTED. Enqueued on `stream`; returns immediately.
+ */
+enum { DL_LOSS_T = 0, DL_LOSS_ALPHA_T = 1, DL_LOSS_SIGMA_T = 2, DL_LOSS_ALPHA_1 = 3, DL_LOSS_SIGMA2_1 = 4,
+       DL_LOSS_LOG_INV_SIGMA_1 = 5, DL_LOSS_COEFS = 6 };
+enum { DL_LOSS_ERROR_T = 0, DL_LOSS_NOISE = 1, DL_LOSS_LOG_P_X = 2, DL_LOSS_LOG_P_H = 3, DL_LOSS_KL_PRIOR = 4,
+       DL_LOSS_N_LINKER = 5, DL_LOSS_TERMS = 6 };
+dl_status dl_diffusion_loss(dl_engine* e, int32_t B, int32_t N, const float* xh, const int8_t* node_mask,
+                            const float* fragment_mask, const float* linker_mask, const int8_t* edge_mask,
+                            const float* context, const float* coef, const float* eps, uint64_t seed, uint64_t offset,
+                            uint64_t* offset_consumed, const float* norm, float* terms, int32_t* nan_flags, void* stream);
 
 dl_status dl_sample_chain_host(dl_engine* e, int32_t sampler, int32_t B, int32_t N, int32_t T, int32_t keep_frames,
                                const float* xh, const int8_t* node_mask, const float* fragment_mask,
